@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- column-iterations/s of the GLOM column update on N B200s (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch: ``Glom.forward(img, iters=12)`` at BASELINE
@@ -26,9 +26,16 @@ Printed (rank 0, ONE JSON line):
   other_configs  BASELINE configs[3] (per-GPU shape) and configs[4] (3-frame continuation), and a training step
   cpu_baseline   the reference's own CPU forward on this box's host cores (bounded sample; rank 0, N = 1 only)
 
-``--impl reference`` times the UNMODIFIED reference package (``$GLOM_REF_PATH`` -> ``baseline/_ref`` ->
-``/root/reference``; torch CPU, all host threads) on the same shapes; if it is not importable on the box it times
-``oracle/glom_oracle_torch.py`` (a torch-CPU restatement pinned on the reference's golden outputs) and says so.
+``--impl reference`` times the UNMODIFIED reference package (``$GLOM_REF_PATH`` -> ``oracle/_ref``; torch CPU, all
+host threads) on the same shapes; if it is not importable on the box it times ``oracle/glom_oracle_torch.py`` (a
+torch-CPU restatement pinned on the reference's golden outputs) and says so.
+
+``--dump-outputs DIR`` writes, after the timed steps, what the last timed step returned (rank 0's shard) as
+``DIR/levels.npy``: float32 ``(columns, levels, dim)`` for a fixed seeded sample of DUMP_COLUMNS (image, patch)
+columns in (image, patch) order, or every column when the batch has no more (<= 50 MB).  Inputs and weights are
+seeded, so two builds run with the same arguments can be compared output for output.
+
+bench.py writes nothing into the tree: a library older than its sources is rebuilt into a temporary directory.
 """
 import argparse
 import json
@@ -37,6 +44,8 @@ import statistics
 import subprocess
 import sys
 import time
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
@@ -49,6 +58,8 @@ N_PATCH = (CFG["image_size"] // CFG["patch_size"]) ** 2
 METRIC = "column-iterations/sec (BxNxLxiters) at dim=512 L=6 224/14"
 UNIT = "column-iterations/s"
 NOMINAL_FLOP_PER_CLK = 148 * 8192.0        # dense bf16: 4096 MAC/clk/SM x 148 SMs (2.25 PFLOP/s at ~1.86 GHz)
+DUMP_COLUMNS = 4096                         # x levels x dim x 4 B = 50 MB at configs[1] (the full state is 100 MB)
+DUMP_SEED = 0
 
 
 def flops_per_col_iter(d, L, n, iters=None):
@@ -95,7 +106,7 @@ def cpu_model_name():
 def find_reference():
     """The unmodified reference package, if importable on this box: (module, where) or (None, why)."""
     tried = []
-    for cand in (os.environ.get("GLOM_REF_PATH"), os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
+    for cand in (os.environ.get("GLOM_REF_PATH"), os.path.join(ROOT, "oracle", "_ref")):
         if not cand or not os.path.isdir(os.path.join(cand, "glom_pytorch")):
             continue
         sys.path.insert(0, cand)
@@ -110,7 +121,7 @@ def find_reference():
         finally:
             if sys.path and sys.path[0] == cand:
                 sys.path.pop(0)
-    return None, "; ".join(tried) or "no glom_pytorch package under $GLOM_REF_PATH, baseline/_ref or /root/reference"
+    return None, "; ".join(tried) or "no glom_pytorch package under $GLOM_REF_PATH or oracle/_ref"
 
 
 class CpuArm:
@@ -367,6 +378,16 @@ class ClockSampler:
 
 
 # ------------------------------------------------------------------------------------ ours
+def sample_columns(levels):
+    """(B, n, L, d) -> (k, L, d): the fixed seeded sample of --dump-outputs, gathered on the device."""
+    import torch
+    cols = levels.reshape(-1, levels.shape[-2], levels.shape[-1])
+    if cols.shape[0] > DUMP_COLUMNS:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(cols.shape[0], DUMP_COLUMNS, replace=False))
+        cols = cols.index_select(0, torch.from_numpy(idx).to(cols.device))
+    return cols.float()
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -382,7 +403,13 @@ def main():
     ap.add_argument("--no-other-configs", action="store_true", help="skip configs[3] / configs[4] / training extras")
     ap.add_argument("--no-train", action="store_true")
     ap.add_argument("--train", action="store_true", help="(kept for compatibility: the training step is timed by default)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned to DIR/levels.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -399,9 +426,16 @@ def main():
     numa = bind_to_gpu_numa(local_rank)       # before torch creates threads / pinned buffers
     import torch
     import torch.distributed as dist
+    from glom_pytorch_b200 import _native
     from glom_pytorch_b200.build import build_library, is_stale
-    if rank == 0 and is_stale():
-        build_library()
+    if "GLOM_B200_LIB" not in os.environ and is_stale():
+        # time the current sources, but build them outside the tree (which may be read-only)
+        import atexit
+        import shutil
+        import tempfile
+        tmp = tempfile.mkdtemp(prefix="glom_b200_bench_")
+        atexit.register(shutil.rmtree, tmp, True)
+        _native.LIB_PATH = build_library(out_dir=tmp)
     distributed = world > 1
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
@@ -411,7 +445,6 @@ def main():
         dist.init_process_group("nccl", rank=rank, world_size=world, device_id=dev)
         dist.barrier(device_ids=[local_rank])
     import glom_pytorch_b200 as G
-    from glom_pytorch_b200 import _native
     from glom_pytorch_b200.sharding import shard_range
 
     if args.warmup < 3:
@@ -480,13 +513,16 @@ def main():
         _native.kernel_clocks(reset=True)        # in-kernel (clock64, %globaltimer) samples of the timed region only
         ev0.record(stream)
         for i in range(args.steps):
-            model(dev_imgs[i % NBUF], iters=T)
+            last = None                          # free the previous result first: the allocator reuses one output block
+            last = model(dev_imgs[i % NBUF], iters=T)
             launches += model.last_launches
         ev1.record(stream)
         enqueue_clock_probe(1)
         barrier()
         ms_dev = ev0.elapsed_time(ev1)
         kernel_clk = _native.kernel_clocks(reset=True)
+        dump = sample_columns(last) if args.dump_outputs and rank == 0 else None   # stays on the device until the end
+        del last
         # -------- the same K steps again, back to back, with CUDA events around EVERY kernel launch (library hook):
         # per-kernel durations for the roofline.  Kept out of the region above because an event between two kernels
         # disables their programmatic (PDL) overlap and costs ~1 us each: the instrumented pass is a few % slower.
@@ -793,6 +829,9 @@ def main():
             line["other_configs"] = other
         if train is not None:
             line["train"] = train
+        if dump is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "levels.npy"), dump.cpu().numpy())
         if world == 1 and not args.no_cpu_baseline:
             # the reference arm's own code path, in a child process with the ORIGINAL CPU affinity (this process and
             # its thread pools are pinned to the GPU's NUMA node), on a bounded sample: 3 timed forwards

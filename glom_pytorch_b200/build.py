@@ -32,14 +32,16 @@ def is_stale():
     return any(os.path.getmtime(d) > t for d in deps if os.path.exists(d))
 
 
-def build_library(force=False, verbose=False):
-    """Compile every CUDA source of the engine into one shared library. Returns its path."""
-    if not force and not is_stale():
+def build_library(force=False, verbose=False, out_dir=None):
+    """Compile every CUDA source of the engine into one shared library. Returns its path.
+    out_dir: write the objects and the library there instead of into the package (always builds)."""
+    if out_dir is None and not force and not is_stale():
         return LIB
+    lib_path = LIB if out_dir is None else os.path.join(out_dir, os.path.basename(LIB))
     objs = []
     procs = []
     for s in SOURCES:
-        o = os.path.join(CSRC, s.replace(".cu", ".o"))
+        o = os.path.join(CSRC if out_dir is None else out_dir, s.replace(".cu", ".o"))
         cmd = [_nvcc(), *NVCC_FLAGS, "-c", os.path.join(CSRC, s), "-o", o]
         if verbose:
             cmd.insert(1, "-Xptxas=-v")
@@ -52,12 +54,12 @@ def build_library(force=False, verbose=False):
         if p.returncode:
             raise RuntimeError(f"nvcc failed on {s}")
     link = [_nvcc(), "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-cudart", "static",
-            "-Xcompiler", "-fPIC", *objs, "-o", LIB]
+            "-Xcompiler", "-fPIC", *objs, "-o", lib_path]
     r = subprocess.run(link, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
     if r.returncode:
         sys.stderr.write(r.stdout)
         raise RuntimeError("nvcc link failed")
-    return LIB
+    return lib_path
 
 
 if __name__ == "__main__":

@@ -4,7 +4,7 @@ Same algorithm and citations as ``oracle/glom_oracle.py`` (the numpy oracle, pin
 outputs), written with batched torch CPU ops (``torch.bmm`` over the MLP groups, ``F.gelu``, ``torch.softmax``) so
 that it uses every host core the way the reference's own torch/oneDNN path does.  ``bench.py`` times it as the CPU
 arm (``kind: "port"``) ONLY when the unmodified reference package is not importable on the box
-(``$GLOM_REF_PATH`` -> ``baseline/_ref`` -> ``/root/reference``); ``tests/test_oracle_golden.py`` checks it against
+(``$GLOM_REF_PATH`` -> ``oracle/_ref``); ``tests/test_oracle_golden.py`` checks it against
 the same golden fixtures as the numpy oracle.  Only ``tests/`` and ``bench.py``'s CPU legs may import this module.
 
 Restates (``glom_pytorch/glom_pytorch.py``): GroupedFeedForward :23-36, ConsensusAttention.forward :56-73

@@ -10,7 +10,7 @@ CASES = {
                              iters=None, return_all=False),
     # mid case (SURVEY 7.1): d=128 L=4 N=64
     "mid_return_all": dict(dim=128, levels=4, image_size=32, patch_size=4, batch=2, iters=5,
-                           return_all=True),
+                           return_all=True, unstored_from=(5, 0, 24, 0, 0)),
     "mid_consensus_self": dict(dim=128, levels=4, image_size=32, patch_size=4, batch=2,
                                iters=3, return_all=False, consensus_self=True),
     "mid_radius": dict(dim=128, levels=4, image_size=32, patch_size=4, batch=2, iters=3,

@@ -63,6 +63,10 @@ def main():
                             levels=None if lv is None else torch.from_numpy(lv),
                             return_all=case["return_all"])
                 outs["out0"] = out.numpy().astype(np.float32)
+        if case.get("unstored_from"):
+            # keeps the fixture under 1 MB: out0 is stored up to the index `unstored_from` (C order) and NaN from there
+            # on (compressed to nothing), so the file keeps the output's full shape
+            outs["out0"].flat[np.ravel_multi_index(case["unstored_from"], outs["out0"].shape):] = np.nan
         np.savez_compressed(os.path.join(HERE, name + ".npz"), **outs)
         index[name] = dict(case=case, shapes={k: list(v.shape) for k, v in outs.items()})
         print(name, {k: v.shape for k, v in outs.items()})

@@ -35,7 +35,7 @@ def test_oracle_matches_reference_golden(name):
             assert np.abs(got - ref).max() <= TOL * scale
             levels = got
     else:
-        got = _run(case, params)
+        got = outs.pick("out0", _run(case, params))
         ref = outs["out0"]
         assert got.shape == ref.shape
         scale = max(1.0, float(np.abs(ref).max()))
@@ -44,7 +44,7 @@ def test_oracle_matches_reference_golden(name):
 
 def test_oracle_fp32_close_to_fp64():
     case, params, outs = load("mid_return_all")
-    a = _run(case, params, dtype=np.float32)
+    a = outs.pick("out0", _run(case, params, dtype=np.float32))
     assert np.abs(a - outs["out0"]).max() <= 1e-4
 
 
@@ -52,7 +52,7 @@ def test_bf16_emulation_within_autocast_gap():
     """The bf16-operand emulation (what the tensor-core engine computes) must stay inside the
     tolerance the GPU parity tests use: rel-Fro <= 1e-2, max-abs <= 3e-2 per time step."""
     case, params, outs = load("mid_return_all")
-    a = _run(case, params, dtype=np.float32, emulate="bf16")
+    a = outs.pick("out0", _run(case, params, dtype=np.float32, emulate="bf16"))
     ref = outs["out0"]
     for t in range(1, ref.shape[0]):
         rel = np.linalg.norm(a[t] - ref[t]) / np.linalg.norm(ref[t])
@@ -108,6 +108,7 @@ def test_torch_cpu_restatement_matches_reference_golden(name):
         img, lv = inputs(case)
         got = OT.glom_forward(params, img, iters=case["iters"], levels=lv, return_all=case.get("return_all", False),
                               **kw).numpy()
+        got = outs.pick("out0", got)
         ref = outs["out0"]
         assert got.shape == ref.shape
         assert np.abs(got - ref).max() <= 1e-4 * max(1.0, float(np.abs(ref).max()))
