@@ -17,9 +17,9 @@ EXPORTS = (
     "glom_b200_profile_begin", "glom_b200_profile_end",
     "glom_b200_backward", "glom_b200_backward_workspace_bytes",
     "glom_b200_tokenize_backward", "glom_b200_tokenize_backward_workspace_bytes",
-    "glom_b200_clock_probe", "glom_b200_mlp_schedule", "glom_b200_islands", "glom_b200_kernel_clocks",
+    "glom_b200_clock_probe", "glom_b200_islands", "glom_b200_kernel_clocks",
 )
-PROFILE_KINDS = ("attention", "gemm1_gelu", "gemm2_combine", "prologue", "tokenize", "mlp_fused")
+PROFILE_KINDS = ("attention", "gemm1_gelu", "gemm2_combine", "prologue", "tokenize")
 
 
 class Cfg(ctypes.Structure):
@@ -77,8 +77,6 @@ def load():
     lib.glom_b200_backward.argtypes = [ctypes.POINTER(Cfg), ctypes.POINTER(WeightsRef), vp, vp, vp, vp,
                                        ctypes.POINTER(Grads), i32, i32, i32, vp, sz, vp]
     lib.glom_b200_backward.restype = i32
-    lib.glom_b200_mlp_schedule.argtypes = [ctypes.POINTER(Cfg), i32, i32, vp, i32, ctypes.POINTER(i32), ctypes.POINTER(i32)]
-    lib.glom_b200_mlp_schedule.restype = i32
     lib.glom_b200_islands.argtypes = [vp, i32, i32, i32, i32, i32, ctypes.c_float, vp, vp, vp, vp, vp, vp]
     lib.glom_b200_islands.restype = i32
     lib.glom_b200_tokenize_backward_workspace_bytes.argtypes = [i32, i32, i32, i32, i32, ctypes.POINTER(sz)]
@@ -221,15 +219,6 @@ def kernel_clocks(reset=True):
     mhz, ms, wf = (ctypes.c_double * k)(), (ctypes.c_double * k)(), (ctypes.c_double * (6 * k))()
     check(load().glom_b200_kernel_clocks(mhz, ms, wf, k, int(bool(reset))))
     return {PROFILE_KINDS[i]: (mhz[i], ms[i], [round(wf[6 * i + j], 4) for j in range(6)]) for i in range(k) if ms[i] > 0}
-
-
-def mlp_schedule(cfg, batch, num_sms=148):
-    """Work list of the merged MLP kernel: (list of (kind, z, m_blk, n_blk), delay).  Host only."""
-    n, dl = ctypes.c_int(), ctypes.c_int()
-    check(load().glom_b200_mlp_schedule(ctypes.byref(cfg), batch, num_sms, None, 0, ctypes.byref(n), ctypes.byref(dl)))
-    buf = (ctypes.c_int32 * (4 * n.value))()
-    check(load().glom_b200_mlp_schedule(ctypes.byref(cfg), batch, num_sms, buf, n.value, ctypes.byref(n), ctypes.byref(dl)))
-    return [tuple(buf[4 * i:4 * i + 4]) for i in range(n.value)], dl.value
 
 
 def islands(states_ptr, slabs, side_h, side_w, levels, dim, threshold, cos_right_ptr, cos_down_ptr, agreement_ptr,

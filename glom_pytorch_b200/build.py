@@ -9,8 +9,8 @@ import sys
 PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libglom_b200.so")
-SOURCES = ["glom_api.cu", "simt_kernels.cu", "tc_kernels.cu", "mlp_kernel.cu", "islands.cu", "bwd_kernels.cu", "tc_bwd_kernels.cu"]
-HEADERS = ["engine.h", "ptx.cuh", "tc_common.cuh", os.path.join("..", "..", "include", "glom_b200.h")]
+SOURCES = ["glom_api.cu", "simt_kernels.cu", "tc_kernels.cu", "islands.cu", "bwd_kernels.cu", "tc_bwd_kernels.cu"]
+HEADERS = ["engine.h", "ptx.cuh", os.path.join("..", "..", "include", "glom_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "-cudart", "static",

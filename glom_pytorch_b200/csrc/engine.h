@@ -12,7 +12,7 @@ namespace glom {
 
 // Optional per-kernel CUDA-event timing (bench.py's roofline numbers).  Events are recorded on the
 // launch stream around each kernel; nothing is synchronised until the caller reads them.
-enum ProfKind { PROF_ATTN = 0, PROF_GEMM1 = 1, PROF_GEMM2 = 2, PROF_PREP = 3, PROF_TOKENIZE = 4, PROF_MLP = 5, PROF_KINDS = 6 };
+enum ProfKind { PROF_ATTN = 0, PROF_GEMM1 = 1, PROF_GEMM2 = 2, PROF_PREP = 3, PROF_TOKENIZE = 4, PROF_KINDS = 5 };
 struct Profiler {
   bool enabled = false;
   std::vector<cudaEvent_t> ev;
@@ -67,8 +67,6 @@ struct WorkspaceLayout {
   size_t nsq_bytes;
   size_t attn_acc_off; // bf16 engine, n > 576 columns: fp32 output / (stabiliser, row sum) carried between the consensus kernel's key passes
   size_t attn_acc_bytes;
-  size_t sched_off;    // bf16 engine, merged MLP kernel: per iteration a tile counter + ready[L * row blocks] (ints)
-  size_t sched_bytes;
   size_t total;
 };
 WorkspaceLayout workspace_layout(const Geometry& g, int precision, int iters, int return_all);
@@ -96,19 +94,12 @@ cudaError_t launch_prep(const Geometry& g, const float* state_in, const float* i
                         const float* tokens, float* s32_dst, __nv_bfloat16* sb, __nv_bfloat16* sp,
                         __nv_bfloat16* xb, float* nsq, cudaStream_t st, int* launches, Profiler* prof);
 
-// one Jacobi step on tensor cores.  sched == nullptr (or dim % 256 != 0): GEMM1+GELU -> H ; consensus -> C ;
-// GEMM2+combine -> state t+1 (three launches).  Otherwise: consensus -> C, then the merged persistent MLP kernel
-// (mlp_kernel.cu; `sched` = this step's zeroed scheduler / dependency counters, mlp_sched_ints(g) ints).
+// one Jacobi step on tensor cores, three launches: GEMM1+GELU -> H ; consensus -> C ; GEMM2+combine -> state t+1.
 // step_index: position of the step inside the forward call.  The bottom-up net of level 0 reads the tokens, which do not
 // change during a call (glom_pytorch.py:132-134), so its hidden activations (MLP group 0 of H) are computed by step 0 only
-// and re-read by GEMM2 of the later steps (three-launch path).
-int step_bf16(const Geometry& g, const Bf16Buffers& b, int* sched, int step_index, EncodeTiledFn enc, int num_sms, cudaStream_t st,
+// and re-read by GEMM2 of the later steps.
+int step_bf16(const Geometry& g, const Bf16Buffers& b, int step_index, EncodeTiledFn enc, int num_sms, cudaStream_t st,
               int* launches, char* err, size_t errlen, Profiler* prof);
-bool mlp_fused_supported(const Geometry& g);
-size_t mlp_sched_ints(const Geometry& g);
-int mlp_schedule_dump(const Geometry& g, int num_sms, int* out, int capacity, int* num_tiles, int* delay);
-int step_bf16_mlp_fused(const Geometry& g, const Bf16Buffers& b, int* sched, EncodeTiledFn enc, int num_sms,
-                        cudaStream_t st, int* launches, char* err, size_t errlen, Profiler* prof);
 
 struct F32Buffers {
   const float* s_in;  float* s_out;
@@ -133,9 +124,8 @@ cudaError_t launch_islands(const float* states, int slabs, int side_h, int side_
                            cudaStream_t st, int* launches);
 
 cudaError_t launch_clock_probe(unsigned long long* out, unsigned long long spin_ns, cudaStream_t st);
-// (cycles, ns) sampled INSIDE the tensor-core kernels since the last reset, by ProfKind (tc_kernels.cu) / merged MLP kernel
+// (cycles, ns) sampled INSIDE the tensor-core kernels since the last reset, by ProfKind (tc_kernels.cu)
 cudaError_t tc_kernel_clocks(unsigned long long* out /* [PROF_KINDS][8] */, bool reset);
-cudaError_t mlp_kernel_clocks(unsigned long long* out /* [2] */, bool reset);
 
 // bf16 tokeniser: patchify + cast (CUDA cores), then the tcgen05 GEMM
 cudaError_t launch_patchify_bf16(const float* img, const float* w, __nv_bfloat16* patches, __nv_bfloat16* wtok, int B,

@@ -61,9 +61,6 @@ WorkspaceLayout workspace_layout(const Geometry& g, int precision, int iters, in
   w.attn_acc_off = off;
   w.attn_acc_bytes = (precision == GLOM_B200_BF16 && g.n > 576) ? (state_elems + (size_t)g.rows * g.L * 2) * 4 : 0;
   off = align_up(off + w.attn_acc_bytes, 1024);
-  w.sched_off = off;
-  w.sched_bytes = (precision == GLOM_B200_BF16 && mlp_fused_supported(g)) ? (size_t)iters * mlp_sched_ints(g) * sizeof(int) : 0;
-  off = align_up(off + w.sched_bytes, 1024);
   w.total = off > 0 ? off : 1024;
   return w;
 }
@@ -117,15 +114,6 @@ static int device_info(DeviceInfo* out) {
     g_dev[dev].ok = (major == 10);
     g_dev[dev].sms = sms;
     g_dev_known[dev] = true;
-    // GLOM_B200_L2_PERSIST_MB (diagnostics): set-aside for L2 lines written / read with an evict-last policy
-    if (const char* pe = getenv("GLOM_B200_L2_PERSIST_MB")) {
-      int maxp = 0;
-      cudaDeviceGetAttribute(&maxp, cudaDevAttrMaxPersistingL2CacheSize, dev);
-      size_t want = (size_t)atoi(pe) << 20;
-      if (want > (size_t)maxp) want = (size_t)maxp;
-      const cudaError_t pe_rc = cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want);
-      fprintf(stderr, "[glom_b200] persisting L2 set-aside: asked %zu MB of max %d MB -> %s\n", want >> 20, maxp >> 20, cudaGetErrorString(pe_rc));
-    }
   }
   if (!g_encode) {
     void* fn = nullptr;
@@ -277,18 +265,6 @@ static int forward_impl(const glom_b200_cfg* cfg, const void* packed_weights, co
                       &g_launches, &g_prof);
     }
     if (e != cudaSuccess) return fail(GLOM_B200_ERR_CUDA, "prep launch: %s", cudaGetErrorString(e));
-    // The step is three launches (GEMM1+GELU, consensus, GEMM2+combine).  GLOM_B200_MERGED_MLP=1 (A/B experiment, kept
-    // bit-identical and tested) replaces the two GEMM launches by the merged persistent MLP kernel (dim % 256 == 0): its
-    // list heads / dependency counters for every step are zeroed once per call.  Measured slower on B200 (profiles/README.md,
-    // r2: H does not survive in L2 between its GEMM1 and GEMM2 tiles), hence opt-in.
-    const char* merged_env = getenv("GLOM_B200_MERGED_MLP");     // read per call: tests toggle it in-process
-    const bool split_mlp = !(merged_env && merged_env[0] == '1');
-    int* sched = nullptr;
-    if (wl.sched_bytes && !split_mlp && iters > 0) {
-      sched = reinterpret_cast<int*>(ws + wl.sched_off);
-      e = cudaMemsetAsync(sched, 0, wl.sched_bytes, st);
-      if (e != cudaSuccess) return fail(GLOM_B200_ERR_CUDA, "scheduler counters memset: %s", cudaGetErrorString(e));
-    }
     for (int t = 0; t < iters; ++t) {
       Bf16Buffers b{};
       b.s32_in = (s0_direct && t == 0) ? (state_in ? state_in : init_levels) : loc(t); b.s32_out = loc(t + 1);
@@ -306,8 +282,7 @@ static int forward_impl(const glom_b200_cfg* cfg, const void* packed_weights, co
       b.b1 = reinterpret_cast<const float*>(pw + pl.b1_off);
       b.b2 = reinterpret_cast<const float*>(pw + pl.b2_off);
       char msg[400] = "";
-      const int r = step_bf16(g, b, sched ? sched + (size_t)t * mlp_sched_ints(g) : nullptr, t, g_encode, di.sms, st,
-                              &g_launches, msg, sizeof(msg), &g_prof);
+      const int r = step_bf16(g, b, t, g_encode, di.sms, st, &g_launches, msg, sizeof(msg), &g_prof);
       if (r) return fail(r == -1 ? GLOM_B200_ERR_INVALID : GLOM_B200_ERR_CUDA, "step %d: %s", t, msg);
     }
   } else {
@@ -465,15 +440,6 @@ GLOM_B200_API int glom_b200_islands(const float* states, int slabs, int side_h, 
   return 0;
 }
 
-GLOM_B200_API int glom_b200_mlp_schedule(const glom_b200_cfg* cfg, int batch, int num_sms, int32_t* out, int capacity,
-                                         int* num_tiles, int* delay) {
-  if (int r = check_cfg(cfg)) return r;
-  if (batch < 1 || num_sms < 2 || capacity < 0 || (capacity > 0 && !out)) return fail(GLOM_B200_ERR_INVALID, "bad arguments");
-  if (mlp_schedule_dump(make_geometry(cfg, batch), num_sms, out, capacity, num_tiles, delay))
-    return fail(GLOM_B200_ERR_INVALID, "the merged MLP kernel needs bf16 precision shapes with dim %% 256 == 0");
-  return 0;
-}
-
 GLOM_B200_API int glom_b200_clock_probe(uint64_t* out_cycles_ns, int spin_us, void* stream) {
   if (!out_cycles_ns || spin_us < 1 || spin_us > 100000) return fail(GLOM_B200_ERR_INVALID, "clock probe: bad arguments");
   cudaError_t e = launch_clock_probe(reinterpret_cast<unsigned long long*>(out_cycles_ns), (unsigned long long)spin_us * 1000ull,
@@ -485,13 +451,9 @@ GLOM_B200_API int glom_b200_clock_probe(uint64_t* out_cycles_ns, int spin_us, vo
 GLOM_B200_API int glom_b200_kernel_clocks(double* mhz_by_kind, double* ms_by_kind, double* wait_frac, int kinds, int reset) {
   if (!mhz_by_kind || !ms_by_kind || kinds < 1) return fail(GLOM_B200_ERR_INVALID, "kernel clocks: bad arguments");
   unsigned long long acc[PROF_KINDS][8];
-  unsigned long long mlp[2];
   cudaError_t e = cudaDeviceSynchronize();
   if (e == cudaSuccess) e = tc_kernel_clocks(&acc[0][0], reset != 0);
-  if (e == cudaSuccess) e = mlp_kernel_clocks(mlp, reset != 0);
   if (e != cudaSuccess) return fail(GLOM_B200_ERR_CUDA, "kernel clocks: %s", cudaGetErrorString(e));
-  for (int j = 0; j < 8; ++j) acc[PROF_MLP][j] = 0;
-  acc[PROF_MLP][0] = mlp[0]; acc[PROF_MLP][1] = mlp[1];
   for (int i = 0; i < kinds; ++i) {
     const bool have = i < PROF_KINDS && acc[i][1] > 0;
     mhz_by_kind[i] = have ? 1e3 * (double)acc[i][0] / (double)acc[i][1] : 0.0;     // cycles per ns -> MHz

@@ -180,32 +180,7 @@ __device__ __forceinline__ uint32_t mapa_shared(uint32_t local_addr, uint32_t ra
 __device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
   asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
 }
-// One 32-bit value into the shared memory of another CTA of the cluster, accounted (4 bytes) on an mbarrier of that
-// CTA: the value is visible to whoever observes the barrier phase complete (st.async carries its own ordering, no
-// cluster-scope release fence is needed).  Both addresses are shared::cluster addresses (mapa_shared).
-__device__ __forceinline__ void st_async_b32(uint32_t cluster_addr, uint32_t value, uint32_t bar_cluster_addr) {
-  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.b32 [%0], %1, [%2];" ::"r"(cluster_addr),
-               "r"(value), "r"(bar_cluster_addr)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx_cluster(uint32_t bar_cluster_addr, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cluster.b64 _, [%0], %1;" ::"r"(bar_cluster_addr), "r"(bytes)
-               : "memory");
-}
-// generic-proxy accesses to global memory <-> async-proxy (TMA) accesses to the same locations
-__device__ __forceinline__ void fence_proxy_async_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
-// counter += v with release semantics at gpu scope: everything that happened before it in this thread -- and, by
-// cumulativity, in threads that synchronised with it (bar.warp.sync, mbarrier) -- is visible to a thread that
-// observes the new value with ld.acquire.gpu.  One MEMBAR.ALL.GPU in the executing thread only.
-__device__ __forceinline__ void red_release_gpu_add(int* p, int v) {
-  asm volatile("red.release.gpu.global.add.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-__device__ __forceinline__ int ld_acquire_gpu(const int* p) {
-  int v;
-  asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
 
 // TMA load into THIS CTA's shared memory whose bytes are accounted on an mbarrier given as a
 // shared::cluster address (the pair leader's barrier).
@@ -232,11 +207,6 @@ __device__ __forceinline__ void tma_load_2d_2sm_sa_hint(uint32_t dst_smem, const
       "l"(m), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "l"(policy)
       : "memory");
 }
-// L2 prefetch of a tensor-map box (no shared-memory destination, no completion tracking): the later TMA load of the same
-// box then hits L2 instead of waiting on HBM
-__device__ __forceinline__ void tma_prefetch_2d(const CUtensorMap* m, int c0, int c1) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global [%0, {%1, %2}];" ::"l"(m), "r"(c0), "r"(c1) : "memory");
-}
 // same with an L2 cache policy (createpolicy value), e.g. evict-first for operands that stream through once
 __device__ __forceinline__ void tma_load_2d_2sm_hint(void* dst, const CUtensorMap* m, uint32_t bar_cluster_addr, int c0,
                                                      int c1, uint64_t policy) {
@@ -245,21 +215,6 @@ __device__ __forceinline__ void tma_load_2d_2sm_hint(void* dst, const CUtensorMa
       "[%0], [%1, {%3, %4}], [%2], %5;" ::"r"(smem_u32(dst)),
       "l"(m), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "l"(policy)
       : "memory");
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_normal() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ void st_global_v4_hint(void* p, uint4 v, uint64_t policy) {
-  asm volatile("st.global.L2::cache_hint.v4.b32 [%0], {%1, %2, %3, %4}, %5;" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w),
-               "l"(policy)
-               : "memory");
 }
 __device__ __forceinline__ uint64_t l2_policy_evict_first() {
   uint64_t pol;

@@ -11,13 +11,18 @@
 // lane), warp 2 = TMEM allocator, remaining warps = TMEM->register epilogue / softmax.  The GEMMs
 // run on CTA pairs (cluster of 2, tcgen05 cta_group::2, UMMA 256 x BN x 16).
 // Operands are staged by TMA into 128B-swizzled shared memory; accumulators live in TMEM.
-#include "tc_common.cuh"
+#include "engine.h"
+#include "ptx.cuh"
 
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 
 namespace glom {
+
+constexpr int BM = 128;            // UMMA M (rows of the state per tile)
+constexpr int BK = 64;             // bf16 elements per 128-byte swizzle row
+constexpr uint32_t A_STAGE_BYTES = BM * BK * 2;   // 16 KB
 
 // =====================================================================================
 // K1 / K2: persistent grouped GEMM on CTA pairs (cta_group::2), fused epilogues
@@ -57,11 +62,6 @@ struct GemmParams {
   // tokeniser (MODE 2)
   float* tok_out;
   int tok_kb;      // K blocks of 64 of the zero-padded patch dimension
-  int h_prefetch;  // K2: k-blocks of H prefetched into L2 ahead of the TMA loads (0 = off)
-  int z_rev;        // K1: groups walked from G - 1 down to z0 (see step_bf16)
-  int h_keep_z;     // K1: H blocks of groups <= h_keep_z are stored with the default L2 policy instead of streaming stores
-  int h_load_policy; // K2: L2 hint of the H loads (GLOM_B200_K2_HPOL, default 0 = evict-first on every load)
-  int epi_prefetch; // K2: L2 prefetch of the epilogue's state / consensus lines at tile start (GLOM_B200_K2_EPI_PREFETCH, default on)
 };
 
 template <int MODE, int BN>
@@ -96,7 +96,7 @@ __device__ __forceinline__ TileInfo decode_tile(const GemmParams& p, int tile) {
   t.n_blk = tile % p.num_n;
   const int r = tile / p.num_n;
   t.m_blk = r % p.num_m;
-  t.z = (MODE == 0 && p.z_rev) ? p.G - 1 - r / p.num_m : p.z0 + r / p.num_m;
+  t.z = p.z0 + r / p.num_m;
   if (MODE == 0) t.num_kb = p.d / BK;
   else if (MODE == 1) t.num_kb = ((t.z == p.L - 1) ? 4 * p.d : 8 * p.d) / BK;   // top level: no top-down half (:137)
   else t.num_kb = p.tok_kb;
@@ -145,6 +145,121 @@ __device__ __forceinline__ int sched_tile(const GemmParams& p, int c, int C, int
   }
   const int j = first + k * C + c;            // the rest: round-robin over all clusters
   return j < S ? B + j : -1;
+}
+
+// Sum of squares of a 32-column chunk row, in the canonical order shared with prep_state_kernel:
+// 8 lanes hold 4 consecutive columns each (sequential fmaf), then an xor tree over the 8 lanes.
+__device__ __forceinline__ float row_chunk_sumsq(float a, float b, float c, float d) {
+  float q = a * a;
+  q = fmaf(b, b, q);
+  q = fmaf(c, c, q);
+  q = fmaf(d, d, q);
+  q += __shfl_xor_sync(0xffffffffu, q, 1);
+  q += __shfl_xor_sync(0xffffffffu, q, 2);
+  q += __shfl_xor_sync(0xffffffffu, q, 4);
+  return q;
+}
+
+// ---- K1 epilogue chunk: 32 rows x 32 columns.  Row-per-thread bias + exact-erf GELU + bf16 pack, transpose
+// through the warp's 2 KB patch (16-byte chunk c of row r stored at chunk c ^ ((r >> 1) & 3)), then 64-byte
+// row segments out (8 rows x 64 B per store instruction).
+template <bool FULL>
+__device__ __forceinline__ void k1_chunk(const uint32_t (&v)[32], const float* bias, uint8_t* patch,
+                                         __nv_bfloat16* hdst /* &H[row0][col] */, size_t pitch, int lane, int rows_left) {
+  uint32_t pk[16];
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    // bias slice read per use (broadcast LDS.128): 32 fewer live registers, so the polynomial's constant pairs stay in
+    // registers instead of being re-materialised for every pair
+    const float4 b = *reinterpret_cast<const float4*>(bias + 4 * i);
+    pk[2 * i] = gelu_pair_bf16(__uint_as_float(v[4 * i + 0]), __uint_as_float(v[4 * i + 1]), b.x, b.y);
+    pk[2 * i + 1] = gelu_pair_bf16(__uint_as_float(v[4 * i + 2]), __uint_as_float(v[4 * i + 3]), b.z, b.w);
+  }
+#pragma unroll
+  for (int c = 0; c < 4; ++c)
+    *reinterpret_cast<uint4*>(patch + lane * 64 + ((c ^ ((lane >> 1) & 3)) << 4)) =
+        make_uint4(pk[4 * c], pk[4 * c + 1], pk[4 * c + 2], pk[4 * c + 3]);
+  __syncwarp();
+  const int c = lane & 3;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int r = i * 8 + (lane >> 2);
+    const uint4 val = *reinterpret_cast<const uint4*>(patch + r * 64 + ((c ^ ((r >> 1) & 3)) << 4));
+    // streaming (evict-first) stores: H (369 MB per step) never fits L2, and letting it through the normal policy
+    // evicts the state shadows and weights the GEMMs and the consensus kernel re-read (measured: K1 -4 %)
+    if (FULL || r < rows_left) __stcs(reinterpret_cast<uint4*>(hdst + (size_t)r * pitch + c * 8), val);
+  }
+  __syncwarp();
+}
+
+// ---- K2 epilogue chunk: the 4-way combine (glom_pytorch.py:141-142) on a 32 x 32 accumulator chunk.
+// The accumulators go through the warp's 4 KB patch (f32, 128-byte rows, chunk c of row r at c ^ (r & 7)) so
+// that each lane then owns 4 consecutive columns of 8 rows and every global access covers whole 128-byte lines.
+struct K2Chunk {
+  int l, L, d, n, row0;
+  int prow0;            // row0 % n: patch index of the band's first row (position table row), computed once per tile
+  int s_bcast;          // 1: s32_in is init_levels (L, d), the same for every row (first step of a call without carried state)
+  const float* s32_in; const __nv_bfloat16* c_in; const float* pos;
+  float* s32_out; __nv_bfloat16* sb_out; __nv_bfloat16* sp_out;
+};
+template <bool FULL>
+__device__ __forceinline__ void k2_chunk(const uint32_t (&v)[32], const float4 b4, uint8_t* patch, const K2Chunk& k,
+                                         int col, int lane, int rows_left, float (&rowsq)[8]) {
+#pragma unroll
+  for (int c = 0; c < 8; ++c)
+    *reinterpret_cast<uint4*>(patch + lane * 128 + ((c ^ (lane & 7)) << 4)) =
+        make_uint4(v[4 * c], v[4 * c + 1], v[4 * c + 2], v[4 * c + 3]);
+  __syncwarp();
+  const int c = lane & 7, rsub = lane >> 3;
+  const bool top = (k.l == k.L - 1);                  // 3 contributions on the top level, 4 elsewhere (:128-129)
+  const bool has_td = (k.l >= 1);
+  const size_t ld = (size_t)k.L * k.d;
+  const size_t base = ((size_t)k.row0 * k.L + k.l) * k.d + col + c * 4;
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    // global loads of four rows first (independent, all in flight), then combine + store
+    float4 sv[4], pp[4];
+    uint2 cw[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int r = (h * 4 + j) * 4 + rsub;
+      sv[j] = make_float4(0.f, 0.f, 0.f, 0.f); pp[j] = sv[j]; cw[j] = make_uint2(0u, 0u);
+      if (FULL || r < rows_left) {
+        sv[j] = k.s_bcast ? __ldg(reinterpret_cast<const float4*>(k.s32_in + (size_t)k.l * k.d + col + c * 4))
+                          : __ldcs(reinterpret_cast<const float4*>(k.s32_in + base + (size_t)r * ld));
+        cw[j] = __ldcs(reinterpret_cast<const uint2*>(k.c_in + base + (size_t)r * ld));
+        if (has_td) {
+          int pr = k.prow0 + r;                       // (row0 + r) % n without a division per row (r < 32)
+          if (k.n >= 32) { if (pr >= k.n) pr -= k.n; } else pr %= k.n;
+          pp[j] = __ldg(reinterpret_cast<const float4*>(k.pos + (size_t)pr * k.d + col + c * 4));
+        }
+      }
+    }
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int i = h * 4 + j;
+      const int r = i * 4 + rsub;
+      const float4 acc = *reinterpret_cast<const float4*>(patch + r * 128 + ((c ^ (r & 7)) << 4));
+      float o0 = (sv[j].x + (acc.x + b4.x)) + __uint_as_float(cw[j].x << 16);               // (:141)
+      float o1 = (sv[j].y + (acc.y + b4.y)) + __uint_as_float(cw[j].x & 0xFFFF0000u);
+      float o2 = (sv[j].z + (acc.z + b4.z)) + __uint_as_float(cw[j].y << 16);
+      float o3 = (sv[j].w + (acc.w + b4.w)) + __uint_as_float(cw[j].y & 0xFFFF0000u);
+      if (top) { o0 = o0 / 3.0f; o1 = o1 / 3.0f; o2 = o2 / 3.0f; o3 = o3 / 3.0f; }          // (:142) IEEE division
+      else { o0 *= 0.25f; o1 *= 0.25f; o2 *= 0.25f; o3 *= 0.25f; }                          // x/4 == x*0.25 exactly
+      if (FULL || r < rows_left) {
+        const size_t o = base + (size_t)r * ld;
+        __stcs(reinterpret_cast<float4*>(k.s32_out + o), make_float4(o0, o1, o2, o3));
+        *reinterpret_cast<uint2*>(k.sb_out + o) = make_uint2(pack_bf16x2(o0, o1), pack_bf16x2(o2, o3));
+        if (has_td)
+          *reinterpret_cast<uint2*>(k.sp_out + ((size_t)(k.row0 + r) * (k.L - 1) + (k.l - 1)) * k.d + col + c * 4) =
+              make_uint2(pack_bf16x2(o0 + pp[j].x, o1 + pp[j].y), pack_bf16x2(o2 + pp[j].z, o3 + pp[j].w));
+      } else {
+        o0 = o1 = o2 = o3 = 0.f;
+      }
+      rowsq[i] += row_chunk_sumsq(o0, o1, o2, o3);
+    }
+  }
+  __syncwarp();
 }
 
 // ---- tokeniser epilogue chunk (image_to_tokens Linear bias, glom_pytorch.py:96): f32 out, whole 128-byte lines.
@@ -234,27 +349,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap map_a0,   // K1: tokens Xb (rows
     const uint64_t pol_first = l2_policy_evict_first();
     const int kbg_n = 4 * p.d / BK;
     const int blk_skip = (p.m128 - 1) * kbg_n;
-    // K2: H comes from HBM (369 MB per step, written by the previous launch); the 5-slot ring covers ~2.5k clk, less
-    // than the loaded HBM latency tail, and the ring is consumed in order.  A cursor running h_prefetch k-blocks ahead
-    // of the loads (across tile boundaries) pulls the 16 KB blocks into L2 first.
-    int pf_it = 0, pf_kb = 0, pf_nkb = 0, pf_blk0 = 0;
-    bool pf_valid = false;
-    auto pf_tile = [&](int it_) {
-      pf_it = it_; pf_kb = 0;
-      const int tl = sched_tile<MODE>(p, cluster_id, num_clusters, it_);
-      pf_valid = tl >= 0;
-      if (pf_valid) {
-        const TileInfo tt = decode_tile<MODE>(p, tl);
-        pf_nkb = tt.num_kb;
-        pf_blk0 = (2 * tt.z * p.m128 + ((tt.m_blk * 256 + (int)cta_rank * BM) >> 7)) * kbg_n;
-      }
-    };
-    auto pf_step = [&]() {
-      if (!pf_valid) return;
-      const int blk = pf_blk0 + pf_kb + (pf_kb >= kbg_n ? blk_skip : 0);
-      if (elected) tma_prefetch_2d(&map_a0, 0, blk * BM);
-      if (++pf_kb == pf_nkb) pf_tile(pf_it + 1);
-    };
     for (int it = 0, tile; (tile = sched_tile<MODE>(p, cluster_id, num_clusters, it)) >= 0; ++it) {
       const TileInfo t = decode_tile<MODE>(p, tile);
       const CUtensorMap* amap;
@@ -277,12 +371,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap map_a0,   // K1: tokens Xb (rows
       // K2: block (group g, 128-row block, 64-wide k block); [H_bu,l | H_td,l] are groups 2l and 2l+1, so k block kb
       // of the concatenation is block blk0 + kb of group 2l and, from kb = kbg_n on, of the group behind it
       const int blk0 = (2 * t.z * p.m128 + (a_row >> 7)) * kbg_n;
-      if (MODE == 1 && it == 0 && p.h_prefetch > 0) {            // prime the prefetch cursor
-        pf_tile(0);
-        for (int i = 0; i < p.h_prefetch; ++i) pf_step();
-      }
       for (int kb = 0; kb < t.num_kb; ++kb) {
-        if (MODE == 1 && p.h_prefetch > 0) pf_step();
         GLOM_CNT_WAIT(w0, mbar_wait(&empty_bar[stage], phase ^ 1));
         if (elected) {
           const uint32_t sa = smem0 + (uint32_t)stage * Cfg::STAGE_BYTES;
@@ -291,9 +380,9 @@ gemm_kernel(const __grid_constant__ CUtensorMap map_a0,   // K1: tokens Xb (rows
           if (MODE == 1) {
             const int blk = blk0 + kb + (kb >= kbg_n ? blk_skip : 0);
             // H streams through once per pair of column tiles: evict-first keeps it from displacing weights / state
-            // (h_load_policy, diagnostics: 1 = only the row block's last column tile marks it evict-first, 2 = no hint)
-            if (p.h_load_policy == 0 || (p.h_load_policy == 1 && t.n_blk == p.num_n - 1)) tma_load_2d_2sm_sa_hint(sa, amap, bar, 0, blk * BM, pol_first);
-            else tma_load_2d_2sm_sa(sa, amap, bar, 0, blk * BM);
+            // (measured best on every load).  An L2 prefetch cursor running ahead of these loads measured slower
+            // (profiles/r2_k2_prefetch_ab.txt).
+            tma_load_2d_2sm_sa_hint(sa, amap, bar, 0, blk * BM, pol_first);
           } else {
             tma_load_2d_2sm_sa(sa, amap, bar, a_col + kb * BK, a_row);
           }
@@ -352,13 +441,12 @@ gemm_kernel(const __grid_constant__ CUtensorMap map_a0,   // K1: tokens Xb (rows
     // swapped in behind a warp barrier -- no CTA-wide barrier, the 16 warps are free to drift apart.  K2 / tokeniser: the
     // 2 x 4 values a lane needs are loaded into registers before the accumulator wait.
     float* bias_w = bias_s + ew * PART_COLS;
-    const uint64_t pol_keep = l2_policy_evict_normal();
     RRIter rr{};
     if (MODE != 1) rr.init(p, cluster_id, num_clusters);
     if (MODE == 0 && rr.tile < p.num_tiles) {
       static_assert(MODE != 0 || PART_COLS == 64, "K1: one float2 of bias per lane");
       *reinterpret_cast<float2*>(bias_w + 2 * lane) =
-          __ldg(reinterpret_cast<const float2*>(p.bias + (size_t)(p.z_rev ? p.G - 1 - rr.z : p.z0 + rr.z) * 4 * p.d + rr.n_blk * BN + part * PART_COLS) + lane);
+          __ldg(reinterpret_cast<const float2*>(p.bias + (size_t)(p.z0 + rr.z) * 4 * p.d + rr.n_blk * BN + part * PART_COLS) + lane);
       __syncwarp();
     }
     for (int it = 0;; ++it) {
@@ -371,11 +459,11 @@ gemm_kernel(const __grid_constant__ CUtensorMap map_a0,   // K1: tokens Xb (rows
         t = decode_tile<MODE>(p, tile);
       } else {
         if (rr.tile >= p.num_tiles) break;
-        t.z = (MODE == 0 && p.z_rev) ? p.G - 1 - rr.z : p.z0 + rr.z; t.m_blk = rr.m_blk; t.n_blk = rr.n_blk; t.num_kb = 0;
+        t.z = p.z0 + rr.z; t.m_blk = rr.m_blk; t.n_blk = rr.n_blk; t.num_kb = 0;
         rr.next(p);                                  // rr now describes the NEXT tile
         has_next = rr.tile < p.num_tiles;
         if (MODE == 0 && has_next)
-          next_bias = __ldg(reinterpret_cast<const float2*>(p.bias + (size_t)(p.z_rev ? p.G - 1 - rr.z : p.z0 + rr.z) * 4 * p.d + rr.n_blk * BN + part * PART_COLS) + lane);
+          next_bias = __ldg(reinterpret_cast<const float2*>(p.bias + (size_t)(p.z0 + rr.z) * 4 * p.d + rr.n_blk * BN + part * PART_COLS) + lane);
       }
       float4 b4r[2] = {make_float4(0.f, 0.f, 0.f, 0.f), make_float4(0.f, 0.f, 0.f, 0.f)};
       if (MODE != 0) {
@@ -385,7 +473,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap map_a0,   // K1: tokens Xb (rows
       }
       const int row0 = t.m_blk * 256 + (int)cta_rank * BM + quad * 32;   // first row of this warp's 32-row band
       const int rows_left = p.rows - row0;                                // >= 32: whole band valid (warp-uniform)
-      if (MODE == 1 && p.epi_prefetch && lane < rows_left) {
+      if (MODE == 1 && lane < rows_left) {
         // The combine reads this warp's 32 x 64 patch of the fp32 state (streamed to HBM by the previous step) and of C:
         // pull those lines into L2 now, a whole main loop (~25 us) before the accumulator is complete, so the epilogue's
         // dependent global loads hit L2 instead of paying the HBM latency four times per tile
@@ -410,10 +498,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap map_a0,   // K1: tokens Xb (rows
           uint32_t v[32];
           tmem_ld32(t_addr + c0, v);
           tmem_ld_wait();
-          if (t.z <= p.h_keep_z) {       // read first by the GEMM2 launch that follows: keep it in L2 if it fits
-            if (rows_left >= 32) k1_chunk<true, 1>(v, bias + c0, patch, hrow + c0, (size_t)BK, lane, 32, pol_keep);
-            else k1_chunk<false, 1>(v, bias + c0, patch, hrow + c0, (size_t)BK, lane, rows_left, pol_keep);
-          } else if (rows_left >= 32) k1_chunk<true>(v, bias + c0, patch, hrow + c0, (size_t)BK, lane, 32);
+          if (rows_left >= 32) k1_chunk<true>(v, bias + c0, patch, hrow + c0, (size_t)BK, lane, 32);
           else k1_chunk<false>(v, bias + c0, patch, hrow + c0, (size_t)BK, lane, rows_left);
         }
       } else if (MODE == 2) {
@@ -1069,6 +1154,30 @@ cudaError_t tc_kernel_clocks(unsigned long long* out /* [PROF_KINDS][8] */, bool
 // =====================================================================================
 // Host side: tensor maps + launches for one Jacobi step
 // =====================================================================================
+static inline bool encode_map(EncodeTiledFn enc, CUtensorMap* m, const void* base, int rank, const uint64_t* dims,
+                       const uint64_t* strides_bytes /* rank-1 */, const uint32_t* box, char* err, size_t errlen,
+                       const char* what) {
+  cuuint64_t gd[3]; cuuint64_t gs[2]; cuuint32_t bx[3]; cuuint32_t es[3] = {1, 1, 1};
+  for (int i = 0; i < rank; ++i) { gd[i] = dims[i]; bx[i] = box[i]; }
+  for (int i = 0; i < rank - 1; ++i) gs[i] = strides_bytes[i];
+  const CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(base), gd, gs, bx, es,
+                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    snprintf(err, errlen, "cuTensorMapEncodeTiled(%s) failed with CUresult %d", what, (int)r);
+    return false;
+  }
+  return true;
+}
+
+static inline bool map2d(EncodeTiledFn enc, CUtensorMap* m, const void* base, uint64_t rows, uint64_t cols, uint32_t box_rows,
+                  char* err, size_t errlen, const char* what) {
+  const uint64_t dims[2] = {cols, rows};
+  const uint64_t strides[1] = {cols * 2};
+  const uint32_t box[2] = {(uint32_t)BK, box_rows};
+  return encode_map(enc, m, base, 2, dims, strides, box, err, errlen, what);
+}
+
 template <int MODE, int BN, bool CNT>
 static cudaError_t launch_gemm_impl(const CUtensorMap& a0, const CUtensorMap& a1, const CUtensorMap& a2, const CUtensorMap& bm,
                                     const GemmParams& p, int num_sms, cudaStream_t st);
@@ -1192,14 +1301,9 @@ static int launch_attention(const Geometry& g, const Bf16Buffers& b, EncodeTiled
   return 0;
 }
 
-int step_bf16(const Geometry& g, const Bf16Buffers& b, int* sched, int step_index, EncodeTiledFn enc, int num_sms, cudaStream_t st,
+int step_bf16(const Geometry& g, const Bf16Buffers& b, int step_index, EncodeTiledFn enc, int num_sms, cudaStream_t st,
               int* launches, char* err, size_t errlen, Profiler* prof) {
   const int d = g.d, L = g.L, n = g.n, rows = g.rows;
-  if (sched && mlp_fused_supported(g)) {
-    // consensus first (reads the state shadow of step t), then ONE persistent kernel for both grouped GEMMs
-    if (int rc = launch_attention(g, b, enc, num_sms, st, launches, err, errlen, prof)) return rc;
-    return step_bf16_mlp_fused(g, b, sched, enc, num_sms, st, launches, err, errlen, prof);
-  }
   // One launch each of K1 (all groups), K3, K2 (all levels).  Splitting K1/K2 into per-level batches so that H stays
   // L2-resident was measured slower (5.3 / 5.6 / 6.5 ms per step for 3 / 2 / 1 levels per batch vs 5.06 ms): the extra
   // kernel boundaries and partial waves cost more than the saved HBM traffic (profiles/README.md).
@@ -1217,18 +1321,10 @@ int step_bf16(const Geometry& g, const Bf16Buffers& b, int* sched, int step_inde
     GemmParams p{};
     p.rows = rows; p.d = d; p.L = L; p.n = n; p.G = g.G;
     // group 0 (bottom-up net of level 0) reads the tokens, which are the same in every step of a call (:132-134): its block
-    // of H is written by the call's first step and stays valid; the later steps run the other 2L - 2 groups only
-    static int reuse_g0 = -1;
-    if (reuse_g0 < 0) { const char* ev = getenv("GLOM_B200_REUSE_BU0"); reuse_g0 = ev ? atoi(ev) : 1; }
-    p.z0 = (step_index > 0 && reuse_g0 && g.G > 1) ? 1 : 0;
-    // Group order: GEMM2 of the previous step wrote the shadows level 0 first, the top level last, and this step's GEMM2
-    // reads H level 0 first.  Walking the groups from the top down reads the most recently written shadows first (L2
-    // hits) and leaves the groups GEMM2 starts with (levels 0, 1) as the last ones written; those are stored with the
-    // default L2 policy instead of streaming stores.  (GLOM_B200_K1_ORDER: bit 0 = reverse walk, bits 1.. = keep groups)
-    static int k1_order = -1;
-    if (k1_order < 0) { const char* ev = getenv("GLOM_B200_K1_ORDER"); k1_order = ev ? atoi(ev) : 0; }
-    p.z_rev = k1_order & 1;
-    p.h_keep_z = (k1_order >> 1) - 1;
+    // of H is written by the call's first step and stays valid; the later steps run the other 2L - 2 groups only.
+    // Groups are walked bottom-up and every H block is a streaming store: a reverse walk and normal-policy stores for
+    // the groups GEMM2 reads first measured no effect (profiles/r2_k1_order_ab.txt).
+    p.z0 = (step_index > 0 && g.G > 1) ? 1 : 0;
     p.num_m = (rows + 255) / 256; p.num_n = 4 * d / 256; p.num_tiles = (g.G - p.z0) * p.num_m * p.num_n;
     p.bias = b.b1; p.h_out = b.h; p.m128 = m128;
     ProfScope scope(prof, PROF_GEMM1, st);
@@ -1248,15 +1344,6 @@ int step_bf16(const Geometry& g, const Bf16Buffers& b, int* sched, int step_inde
     p.m128 = m128;
     p.bias = b.b2; p.s32_in = b.s32_in; p.s_bcast = b.s32_in_bcast; p.c_in = b.c; p.pos = b.pos;
     p.s32_out = b.s32_out; p.sb_out = b.sb_out; p.sp_out = b.sp_out; p.nsq_out = b.nsq_out; p.nparts = g.nparts;
-    static int h_pf = -1;
-    if (h_pf < 0) { const char* ev = getenv("GLOM_B200_K2_PREFETCH"); h_pf = ev ? atoi(ev) : 0; }
-    p.h_prefetch = h_pf;
-    static int epi_pf = -1;
-    if (epi_pf < 0) { const char* ev = getenv("GLOM_B200_K2_EPI_PREFETCH"); epi_pf = ev ? atoi(ev) : 1; }
-    p.epi_prefetch = epi_pf;
-    static int k2_hpol = -1;
-    if (k2_hpol < 0) { const char* ev = getenv("GLOM_B200_K2_HPOL"); k2_hpol = ev ? atoi(ev) : 0; }
-    p.h_load_policy = k2_hpol;
     cudaError_t e;
     ProfScope scope(prof, PROF_GEMM2, st);
     if (g.bn2 == 256) e = launch_gemm<1, 256>(mh, mh, mh, mw2, p, num_sms, st);

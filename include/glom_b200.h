@@ -182,11 +182,9 @@ GLOM_B200_API int glom_b200_tokenize_backward(const float* img, const float* wei
  * kernel the forward/tokenize calls of THIS thread enqueue is bracketed by CUDA events on the
  * launch stream (no synchronisation is added to the calls).  _end waits for those events and
  * returns summed milliseconds and launch counts per kernel kind:
- *   0 consensus attention, 1 GEMM1+GELU, 2 GEMM2+combine, 3 state prologue, 4 tokeniser,
- *   5 merged persistent MLP kernel (GEMM1+GELU and GEMM2+combine tiles of one step in one launch; only with the
- *     environment variable GLOM_B200_MERGED_MLP=1 and dim % 256 == 0 -- the default step is three launches).
+ *   0 consensus attention, 1 GEMM1+GELU, 2 GEMM2+combine, 3 state prologue, 4 tokeniser.
  * `kinds` is the capacity of both arrays (>= 5; kinds beyond the capacity are dropped). */
-#define GLOM_B200_PROFILE_KINDS 6
+#define GLOM_B200_PROFILE_KINDS 5
 GLOM_B200_API int glom_b200_profile_begin(void);
 GLOM_B200_API int glom_b200_profile_end(double* ms_by_kind, int* launches_by_kind, int kinds);
 
@@ -204,15 +202,6 @@ GLOM_B200_API int glom_b200_islands(const float* states, int slabs, int side_h, 
                                     float* cos_right, float* cos_down, float* agreement, int32_t* labels,
                                     int32_t* num_islands, void* stream);
 
-/* Diagnostics (host only, no GPU needed): the two ordered work lists of the merged persistent MLP kernel (opt-in,
- * dim % 256 == 0) for (cfg, batch) on a device with `num_sms` SMs, the GEMM1 list followed by the GEMM2 list, as
- * (kind, z, m_blk, n_blk) quadruples: kind 0 = GEMM1+GELU tile of MLP group z (2l = bottom-up l, 2l+1 = top-down l),
- * kind 1 = GEMM2+combine tile of level z; m_blk = 256-row block, n_blk = 256-column block.  Writes
- * min(capacity, *num_tiles) entries; *delay = row blocks by which the GEMM1 list's head must lead the GEMM2 list's head
- * before a cluster coming from a GEMM1 tile takes the GEMM2 head.  Tests check that both lists are complete. */
-GLOM_B200_API int glom_b200_mlp_schedule(const glom_b200_cfg* cfg, int batch, int num_sms, int32_t* out, int capacity,
-                                         int* num_tiles, int* delay);
-
 /* Measurement aid (bench.py): one device thread spins for `spin_us` microseconds of %globaltimer and writes
  * {SM cycles elapsed, nanoseconds elapsed} to out_cycles_ns[0..1] (device memory, 16 bytes): cycles / ns is the SM
  * clock in GHz the device actually ran at when the probe executed.  Enqueued on `stream`; the caller synchronises. */
@@ -220,7 +209,7 @@ GLOM_B200_API int glom_b200_clock_probe(uint64_t* out_cycles_ns, int spin_us, vo
 
 /* Measurement aid (bench.py): the SM clock the tensor-core kernels ACTUALLY ran at.  One thread of block 0 of every
  * tcgen05 kernel brackets the kernel's working phase with (clock64, %globaltimer); the deltas accumulate per kernel kind
- * (indices as in glom_b200_profile_end: 0 consensus, 1 GEMM1+GELU, 2 GEMM2+combine, 4 tokeniser GEMM, 5 merged MLP kernel).
+ * (indices as in glom_b200_profile_end: 0 consensus, 1 GEMM1+GELU, 2 GEMM2+combine, 4 tokeniser GEMM).
  * Writes MHz (cycles per microsecond of in-kernel time) and the in-kernel milliseconds per kind since the last reset;
  * kinds without samples report 0.  wait_frac (may be NULL, else 6 doubles per kind): fractions of block 0's in-kernel
  * cycles that {the MMA lane waited for operands, the MMA lane waited for a free accumulator stage (consensus: TMEM buffer

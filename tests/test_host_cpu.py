@@ -131,33 +131,6 @@ def test_batch_sharding_two_ranks_gloo():
     assert err <= 1e-4 and tmax == 2.0
 
 
-@pytest.mark.parametrize("dim,L,n,batch,sms", [(512, 6, 256, 32, 148), (1024, 8, 576, 8, 148), (256, 2, 64, 3, 148),
-                                               (512, 3, 16, 1, 148), (512, 6, 256, 5, 20), (768, 4, 100, 7, 132)])
-def test_merged_mlp_kernel_work_list_is_complete_and_ordered(dim, L, n, batch, sms):
-    """Host logic of mlp_kernel.cu: every GEMM1 tile (group, row block, column tile) and every GEMM2 tile (level, row
-    block, column tile) appears exactly once, and each GEMM2 tile comes after all GEMM1 tiles of its (level, row block)
-    -- the property that makes in-order hand-out of the list deadlock-free."""
-    cfg = _native.make_cfg(dim, L, n, False, 0, 0, "bf16")
-    tiles, delay = _native.mlp_schedule(cfg, batch, sms)
-    num_m = (batch * n + 255) // 256
-    nN1, nN2 = 4 * dim // 256, dim // 256
-    want1 = {(g, m, j) for g in range(2 * L - 1) for m in range(num_m) for j in range(nN1)}
-    want2 = {(l, m, j) for l in range(L) for m in range(num_m) for j in range(nN2)}
-    got1 = [(z, m, j) for k, z, m, j in tiles if k == 0]
-    got2 = [(z, m, j) for k, z, m, j in tiles if k == 1]
-    assert len(got1) == len(want1) and set(got1) == want1
-    assert len(got2) == len(want2) and set(got2) == want2
-    assert delay >= 1
-    done = {}
-    for k, z, m, j in tiles:
-        if k == 0:
-            done[(z // 2, m)] = done.get((z // 2, m), 0) + 1
-        else:
-            assert done.get((z, m), 0) == (1 if z == L - 1 else 2) * nN1, (z, m)
-    # the top level (half-cost GEMM2 tiles) closes the list
-    assert tiles[-1][0] == 1 and tiles[-1][1] == L - 1
-
-
 def _dp_worker(rank, world, port, q):
     import torch.distributed as dist
     from glom_pytorch_b200.dp import allreduce_gradients, broadcast_parameters

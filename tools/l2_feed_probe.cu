@@ -5,7 +5,7 @@
 // producer side ALONE: every SM streams 16 KB boxes of an L2-resident bf16 matrix into a 5-slot shared-memory ring
 // (cp.async.bulk.tensor.2d, 128B swizzle, mbarrier completion; a consumer lane frees the slots immediately) and
 // reports bytes per SM clock per SM, chip-wide.  Variants:
-//   unicast       every CTA loads its own 32 KB per stage (what gemm_kernel / mlp_kernel do: A box + half-B box)
+//   unicast       every CTA loads its own 32 KB per stage (what gemm_kernel does: A box + half-B box)
 //   multicast x2  clusters of 2: each CTA loads 16 KB and multicasts it to both CTAs (both receive 32 KB per stage, the
 //                 L2 serves 16 KB per CTA): the cost of DELIVERED bytes when half of them are shared
 //   multicast x4  clusters of 4, each CTA loads 8 KB, multicast to all four

@@ -3,7 +3,7 @@
 //
 // umma_probe.cu shows the tensor pipe sustains 4096 MAC/clk/SM from resident operands, l2_feed_probe.cu that the L2
 // delivers 73 B/clk/SM into all shared memories at once (the main loop needs 64).  This probe runs both together,
-// exactly as gemm_kernel / mlp_kernel do (5-slot ring of 32 KB per CTA, producer lane + MMA lane, mbarrier full / empty
+// exactly as gemm_kernel does (5-slot ring of 32 KB per CTA, producer lane + MMA lane, mbarrier full / empty
 // pairs, tcgen05.commit frees the slot), with NO epilogue: accumulators are simply overwritten.  What is left between
 // this number and the real kernels is the epilogue (TMEM read-out, GELU / combine math, transposes through shared
 // memory, global stores); what is left between this number and 4096 is contention between TMA writes and UMMA reads

@@ -5,7 +5,7 @@
 // accumulate in TMEM) over operands that already sit in 128B-swizzled shared memory (a ring of 4 k-blocks, contents
 // irrelevant), commits to an mbarrier and waits; MACs per SM clock per SM are reported per shape:
 //
-//   cg2 M256 N256 SS   the 256 x 256 CTA-pair tile of gemm_kernel / mlp_kernel                      (reference point)
+//   cg2 M256 N256 SS   the 256 x 256 CTA-pair tile of gemm_kernel                                   (reference point)
 //   cg2 M256 N128 SS   a pair tile with a 128-wide accumulator (what a TMEM budget of Y + H-chunk forces)
 //   cg1 M128 N256 SS   one CTA per 128 rows, d_out split across the pair (the DSMEM-exchange design of SURVEY 7.3)
 //   cg1 M128 N128 SS   ... with 128-wide hidden chunks
