@@ -1,10 +1,13 @@
 """Pin the CPU oracle against every golden vector produced by the live reference
 (tests/golden/make_golden.py).  fp64 oracle vs fp32 reference: <= 2e-5 max-abs relative
 to the state scale (the reference itself is only fp32-accurate)."""
+import os
+
 import numpy as np
 import pytest
 
-from golden_util import CASES, inputs, load
+from cases import GRAD_CASES, grad_inputs
+from golden_util import CASES, GOLDEN_DIR, inputs, load
 from oracle import glom_oracle as O
 
 TOL = 2e-5
@@ -112,3 +115,40 @@ def test_torch_cpu_restatement_matches_reference_golden(name):
         ref = outs["out0"]
         assert got.shape == ref.shape
         assert np.abs(got - ref).max() <= 1e-4 * max(1.0, float(np.abs(ref).max()))
+
+
+@pytest.mark.parametrize("name", sorted(GRAD_CASES))
+def test_fp64_backward_reference_matches_reference_autograd(name):
+    """oracle/glom_oracle_torch.py's gradient reference (fp64 autograd through one column_step per time step, walked
+    backwards along its own fp64 forward, then the tokenizer's VJP) against the reference's autograd
+    (tests/golden/make_golden_grads.py, same seeds): every stored gradient within 1e-6 * max(1, |ref|max)."""
+    import torch
+    from oracle import glom_oracle_torch as OT
+    case = GRAD_CASES[name]
+    with np.load(os.path.join(GOLDEN_DIR, name + ".npz")) as z:
+        ref = {k: z[k] for k in z.files}
+    params = O.synth_params(case["dim"], case["levels"], case["image_size"], case["patch_size"], seed=case["param_seed"])
+    P = {k: torch.from_numpy(v).double() for k, v in params.items()}
+    img, lv, cot = grad_inputs(case)
+    cs, radius = case.get("consensus_self", False), case.get("local_consensus_radius", 0)
+    states = OT.glom_forward(params, img, patch_size=case["patch_size"], iters=case["iters"], levels=lv,
+                             return_all=True, consensus_self=cs, local_consensus_radius=radius, dtype=torch.float64)
+    tokens = OT.tokenize(torch.from_numpy(img).double(), P["image_to_tokens.1.weight"], P["image_to_tokens.1.bias"],
+                         case["patch_size"])
+    mask = OT.radius_mask(case["image_size"] // case["patch_size"], radius) if radius > 0 else None
+    got = OT.reference_grads(P, img, case["patch_size"], states, tokens, P["pos_emb.weight"][:tokens.shape[1]],
+                             torch.from_numpy(cot), return_all=case["return_all"], consensus_self=cs, mask=mask,
+                             carried_levels=lv is not None)
+    checked = 0
+    for k, r in ref.items():
+        if k == "out":
+            continue
+        g = got.get(k[2:])
+        if g is None:                           # init_levels when `levels` is carried in: no gradient reaches it
+            assert k == "d_init_levels" and lv is not None and not r.any(), k
+            continue
+        g = g.numpy()
+        assert g.shape == r.shape, (k, g.shape, r.shape)
+        assert np.abs(g - r).max() <= 1e-6 * max(1.0, float(np.abs(r).max())), (k, np.abs(g - r).max())
+        checked += 1
+    assert checked == len(got)

@@ -1,53 +1,49 @@
-"""Randomised shape sweep of the tensor-core backward (bf16 engine) against the fp32 CUDA-core backward."""
-import os, sys
-import numpy as np, torch
-sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-import glom_pytorch_b200 as G
+"""Randomised shape sweep of the engine's backward against the fp64 reference along the saved forward states.
+
+    python tools/fuzz_grads.py [seed] [cases]
+
+Uses the comparator of tests/test_backward_reference.py (``check`` at that file's thresholds for the path each case
+takes), so the sweep and the suite judge a gradient the same way."""
+import os
+import sys
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+from test_backward_reference import (C, check, engine_and_reference, make_inputs, make_model, path,  # noqa: E402
+                                     report, tolerances)
 
 rng = np.random.default_rng(int(sys.argv[1]) if len(sys.argv) > 1 else 0)
 N = int(sys.argv[2]) if len(sys.argv) > 2 else 14
 bad = 0
 for it in range(N):
-    dim = int(rng.choice([256, 512]))
+    prec = "fp32" if rng.random() < 0.2 else "bf16"
+    dim = int(rng.choice([192, 256, 512]))
     L = int(rng.integers(2, 5))
     p = 2
     side = int(rng.choice([2, 3, 8, 10, 11, 16, 18, 20, 26, 28]))     # 26, 28: n = 676 / 784 > 576 columns
-    if side >= 26: dim = 256
-    B = int(rng.integers(1, 4)); T = int(rng.integers(1, 3))
-    kw = {}
-    if rng.random() < 0.3: kw["consensus_self"] = True
-    if rng.random() < 0.3: kw["local_consensus_radius"] = float(rng.choice([1.5, 2.5]))
-    isz = side * p; n = side * side
+    if side >= 26:
+        dim = min(dim, 256)
+    B = int(rng.integers(1, 4))
+    T = int(rng.integers(1, 3))
+    radius = float(rng.choice([1.5, 2.5])) if rng.random() < 0.3 else 0.0
+    case = C(f"[{it}]", prec, dim, L, side * p, p, B, T, return_all=bool(rng.random() < 0.5),
+             levels=bool(rng.random() < 0.5), consensus_self=bool(rng.random() < 0.3), radius=radius)
     seed = int(rng.integers(1 << 30))
-    ms = {}
-    for prec in ("fp32", "bf16"):
-        torch.manual_seed(seed)
-        ms[prec] = G.Glom(dim=dim, levels=L, image_size=isz, patch_size=p, precision=prec, **kw).cuda()
-    g = torch.Generator().manual_seed(seed)
-    img = torch.randn(B, 3, isz, isz, generator=g).cuda()
-    ra = bool(rng.random() < 0.5)
-    with_lv = bool(rng.random() < 0.5)
-    lv = torch.randn(B, n, L, dim, generator=g).cuda() if with_lv else None
-    cot = torch.randn(((T + 1,) if ra else ()) + (B, n, L, dim), generator=g).cuda()
-    grads = {}
+    tag = (f"[{it}] {prec} d={dim} L={L} n={case['n']} rows={B * case['n']} B={B} T={T} all={case['return_all']} "
+           f"lv={case['levels']} self={case['consensus_self']} radius={radius} [{path(case)}]")
     try:
-        for prec, m in ms.items():
-            x = img.clone().requires_grad_(True)
-            l0 = None if lv is None else lv.clone().requires_grad_(True)
-            out = m(x, iters=T, levels=l0, return_all=ra)
-            (out * cot).sum().backward()
-            grads[prec] = {"img": x.grad, **({"levels": l0.grad} if l0 is not None else {}),
-                           **{k: q.grad for k, q in m.named_parameters()}}
-        torch.cuda.synchronize()
+        m, params = make_model(case, seed)
+        got, ref = engine_and_reference(m, params, case, *make_inputs(case, seed))
     except Exception as e:
-        print(f"[{it}] d={dim} L={L} n={n} B={B} T={T} {kw} EXC {type(e).__name__}: {str(e)[:100]}"); bad += 1; continue
-    worst = ("", 0.0)
-    for k, ref in grads["fp32"].items():
-        got = grads["bf16"][k]
-        if ref is None: continue
-        rel = (torch.linalg.norm(got - ref) / torch.linalg.norm(ref).clamp_min(1e-30)).item()
-        if not np.isfinite(rel) or rel > worst[1]: worst = (k, rel)
-    ok = np.isfinite(worst[1]) and worst[1] <= 3e-2
-    bad += (not ok)
-    print(f"[{it}] d={dim} L={L} n={n} rows={B*n} B={B} T={T} all={ra} lv={with_lv} {kw}: worst rel {worst[1]:.2e} ({worst[0]}) {'ok' if ok else 'FAIL'}", flush=True)
+        print(f"{tag}: EXC {type(e).__name__}: {str(e)[:100]}", flush=True)
+        bad += 1
+        continue
+    failures, worst = check(got, ref, L, dim, **tolerances(case))
+    report(tag, worst)
+    for f in failures[:5]:
+        print("   ", f)
+    bad += bool(failures)
 print("FAILURES:", bad)
