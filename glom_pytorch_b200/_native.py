@@ -18,6 +18,7 @@ EXPORTS = (
     "glom_b200_backward", "glom_b200_backward_workspace_bytes",
     "glom_b200_tokenize_backward", "glom_b200_tokenize_backward_workspace_bytes",
     "glom_b200_clock_probe", "glom_b200_islands", "glom_b200_kernel_clocks",
+    "glom_b200_contrastive_workspace_bytes", "glom_b200_contrastive_forward", "glom_b200_contrastive_backward",
 )
 PROFILE_KINDS = ("attention", "gemm1_gelu", "gemm2_combine", "prologue", "tokenize")
 
@@ -37,6 +38,16 @@ class Grads(ctypes.Structure):
     _fields_ = [("struct_size", ctypes.c_uint32)] + [
         (k, ctypes.c_void_p) for k in ("d_tokens", "d_pos", "d_state0", "d_init", "d_bu_w1", "d_bu_b1", "d_bu_w2",
                                        "d_bu_b2", "d_td_w1", "d_td_b1", "d_td_w2", "d_td_b2")]
+
+
+CONTRASTIVE_MAX_LEVELS = 32
+
+
+class ContrastiveCfg(ctypes.Structure):
+    _fields_ = [("struct_size", ctypes.c_uint32), ("batch", ctypes.c_int32), ("n", ctypes.c_int32),
+                ("levels", ctypes.c_int32), ("dim", ctypes.c_int32), ("num_selected", ctypes.c_int32),
+                ("selected", ctypes.c_int32 * CONTRASTIVE_MAX_LEVELS), ("temperature", ctypes.c_float),
+                ("stride_a", ctypes.c_int64 * 3), ("stride_b", ctypes.c_int64 * 3)]
 
 
 class GlomB200Error(RuntimeError):
@@ -90,6 +101,13 @@ def load():
     lib.glom_b200_clock_probe.restype = i32
     lib.glom_b200_kernel_clocks.argtypes = [vp, vp, vp, i32, i32]
     lib.glom_b200_kernel_clocks.restype = i32
+    cc = ctypes.POINTER(ContrastiveCfg)
+    lib.glom_b200_contrastive_workspace_bytes.argtypes = [cc, ctypes.POINTER(sz), ctypes.POINTER(sz)]
+    lib.glom_b200_contrastive_workspace_bytes.restype = i32
+    lib.glom_b200_contrastive_forward.argtypes = [cc, vp, vp, vp, vp, sz, vp, sz, vp]
+    lib.glom_b200_contrastive_forward.restype = i32
+    lib.glom_b200_contrastive_backward.argtypes = [cc, vp, vp, vp, vp, sz, vp, vp, vp]
+    lib.glom_b200_contrastive_backward.restype = i32
     for f in ("glom_b200_packed_weight_bytes", "glom_b200_pack_weights", "glom_b200_workspace_bytes",
               "glom_b200_workspace_offset", "glom_b200_forward", "glom_b200_tokenize"):
         getattr(lib, f).restype = i32
@@ -225,3 +243,29 @@ def islands(states_ptr, slabs, side_h, side_w, levels, dim, threshold, cos_right
             labels_ptr, num_islands_ptr, stream):
     check(load().glom_b200_islands(states_ptr, slabs, side_h, side_w, levels, dim, threshold, cos_right_ptr, cos_down_ptr,
                                    agreement_ptr, labels_ptr, num_islands_ptr, stream))
+
+
+def make_contrastive_cfg(batch, n, levels, dim, selected, temperature, stride_a, stride_b):
+    """stride_a / stride_b: element strides of the two (B, n, L, d) inputs over (B, n, L)."""
+    if len(selected) > CONTRASTIVE_MAX_LEVELS:
+        raise ValueError(f"at most {CONTRASTIVE_MAX_LEVELS} levels can be selected")
+    sel = (ctypes.c_int32 * CONTRASTIVE_MAX_LEVELS)(*selected)
+    return ContrastiveCfg(ctypes.sizeof(ContrastiveCfg), batch, n, levels, dim, len(selected), sel, float(temperature),
+                          (ctypes.c_int64 * 3)(*stride_a), (ctypes.c_int64 * 3)(*stride_b))
+
+
+def contrastive_workspace_bytes(cfg):
+    """-> (saved bytes, scratch bytes) of glom_b200_contrastive_forward."""
+    saved, scratch = ctypes.c_size_t(), ctypes.c_size_t()
+    check(load().glom_b200_contrastive_workspace_bytes(ctypes.byref(cfg), ctypes.byref(saved), ctypes.byref(scratch)))
+    return saved.value, scratch.value
+
+
+def contrastive_forward(cfg, za_ptr, zb_ptr, loss_ptr, saved_ptr, saved_bytes, scratch_ptr, scratch_bytes, stream):
+    check(load().glom_b200_contrastive_forward(ctypes.byref(cfg), za_ptr, zb_ptr, loss_ptr, saved_ptr, saved_bytes,
+                                               scratch_ptr, scratch_bytes, stream))
+
+
+def contrastive_backward(cfg, za_ptr, zb_ptr, grad_loss_ptr, saved_ptr, saved_bytes, dza_ptr, dzb_ptr, stream):
+    check(load().glom_b200_contrastive_backward(ctypes.byref(cfg), za_ptr, zb_ptr, grad_loss_ptr, saved_ptr, saved_bytes,
+                                                dza_ptr, dzb_ptr, stream))

@@ -9,7 +9,8 @@ import sys
 PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libglom_b200.so")
-SOURCES = ["glom_api.cu", "simt_kernels.cu", "tc_kernels.cu", "islands.cu", "bwd_kernels.cu", "tc_bwd_kernels.cu"]
+SOURCES = ["glom_api.cu", "simt_kernels.cu", "tc_kernels.cu", "islands.cu", "bwd_kernels.cu", "tc_bwd_kernels.cu",
+           "contrastive.cu"]
 HEADERS = ["engine.h", "ptx.cuh", os.path.join("..", "..", "include", "glom_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

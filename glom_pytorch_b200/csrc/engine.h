@@ -181,6 +181,29 @@ cudaError_t tokenize_backward(const float* img, const float* weight, const float
 int backward_run(const Geometry& g, const BackwardArgs& a, int precision, int iters, int grad_all, void* workspace,
                  EncodeTiledFn enc, int num_sms, cudaStream_t st, int* launches, char* err, size_t errlen);
 
+// ---- column-contrastive loss (contrastive.cu) ------------------------------------------------------------
+#define GLOM_CT_MAX_SEL 32      // selected levels per call
+#define GLOM_CT_MAX_SPLIT 8     // column splits of the lse kernel (partial sums in the scratch buffer)
+struct ContrastiveStrides { long long b, n, l; };   // element strides of a (B, n, L, d) input whose d is contiguous
+struct ContrastiveGeom {
+  int R, Rp, n, d, L, nsel;     // R = B n rows per level, Rp = R rounded up to 128
+  int sel[GLOM_CT_MAX_SEL];
+  float tau;
+  ContrastiveStrides sa, sb;
+};
+struct ContrastiveLayout {
+  // saved for the backward: bf16 unit rows A, B (nsel, R, d); fp32 per row (nsel, Rp): 1/|z_a|, 1/|z_b|, the lse of both
+  // directions (log2 units, relative to 1/tau) and G_rr - 1
+  size_t a_off, b_off, inv_a_off, inv_b_off, m_a_off, m_b_off, dg_off, saved;
+  // forward scratch: lse partial sums [GLOM_CT_MAX_SPLIT][nsel][Rp] per direction, s_rr, loss block partials
+  size_t ea_off, eb_off, srr_off, part_off, scratch;
+};
+ContrastiveLayout contrastive_layout(const ContrastiveGeom& g);
+int contrastive_forward(const ContrastiveGeom& g, const float* za, const float* zb, float* loss, void* saved, void* scratch,
+                        EncodeTiledFn enc, int num_sms, cudaStream_t st, int* launches, char* err, size_t errlen);
+int contrastive_backward(const ContrastiveGeom& g, const float* za, const float* zb, const float* grad_loss, const void* saved,
+                         float* dza, float* dzb, EncodeTiledFn enc, cudaStream_t st, int* launches, char* err, size_t errlen);
+
 // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) is per device and per function: remember, per device, the
 // largest size already configured for one kernel (one instance of this per kernel template instantiation).
 struct SmemOptIn {

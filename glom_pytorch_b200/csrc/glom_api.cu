@@ -440,6 +440,104 @@ GLOM_B200_API int glom_b200_islands(const float* states, int slabs, int side_h, 
   return 0;
 }
 
+static_assert(GLOM_B200_CONTRASTIVE_MAX_LEVELS == GLOM_CT_MAX_SEL, "selected-level capacity of the ABI and the kernels");
+
+// The tensor-map encoder is a driver call and needs a current context.  A thread whose first CUDA work is this call (the
+// autograd engine's worker thread running the backward) has none yet: cudaSetDevice makes the primary context current.
+static int bind_current_device() {
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e == cudaSuccess) e = cudaSetDevice(dev);
+  if (e != cudaSuccess) return fail(GLOM_B200_ERR_CUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
+  return 0;
+}
+
+static int contrastive_geometry(const glom_b200_contrastive_cfg* cfg, ContrastiveGeom* g) {
+  if (!cfg) return fail(GLOM_B200_ERR_INVALID, "contrastive cfg is NULL");
+  if (cfg->struct_size != sizeof(glom_b200_contrastive_cfg))
+    return fail(GLOM_B200_ERR_INVALID, "contrastive cfg.struct_size %u != %zu (ABI mismatch)", cfg->struct_size,
+                sizeof(glom_b200_contrastive_cfg));
+  if (cfg->batch < 1 || cfg->n < 1 || cfg->levels < 1)
+    return fail(GLOM_B200_ERR_INVALID, "contrastive: batch, n, levels must be >= 1");
+  if (cfg->dim < 64 || cfg->dim % 64)
+    return fail(GLOM_B200_ERR_INVALID, "contrastive: dim must be a positive multiple of 64 (tcgen05 operands), got %d", cfg->dim);
+  const long long rows = (long long)cfg->batch * cfg->n;
+  if (rows > (1LL << 30)) return fail(GLOM_B200_ERR_INVALID, "contrastive: batch * n = %lld rows is too many", rows);
+  if (!(cfg->temperature >= 0.03f))
+    return fail(GLOM_B200_ERR_INVALID, "contrastive: temperature must be >= 0.03 (got %g)", (double)cfg->temperature);
+  if (cfg->num_selected < 1 || cfg->num_selected > GLOM_B200_CONTRASTIVE_MAX_LEVELS)
+    return fail(GLOM_B200_ERR_INVALID, "contrastive: 1 <= num_selected <= %d", GLOM_B200_CONTRASTIVE_MAX_LEVELS);
+  g->R = (int)rows;
+  g->Rp = (int)((rows + 127) / 128 * 128);
+  g->n = cfg->n; g->d = cfg->dim; g->L = cfg->levels; g->nsel = cfg->num_selected; g->tau = cfg->temperature;
+  for (int i = 0; i < g->nsel; ++i) {
+    const int l = cfg->selected[i];
+    if (l < 0 || l >= cfg->levels) return fail(GLOM_B200_ERR_INVALID, "contrastive: level %d out of range [0, %d)", l, cfg->levels);
+    for (int j = 0; j < i; ++j)
+      if (cfg->selected[j] == l) return fail(GLOM_B200_ERR_INVALID, "contrastive: level %d selected twice", l);
+    g->sel[i] = l;
+  }
+  g->sa = {cfg->stride_a[0], cfg->stride_a[1], cfg->stride_a[2]};
+  g->sb = {cfg->stride_b[0], cfg->stride_b[1], cfg->stride_b[2]};
+  return 0;
+}
+
+GLOM_B200_API int glom_b200_contrastive_workspace_bytes(const glom_b200_contrastive_cfg* cfg, size_t* saved_bytes,
+                                                        size_t* scratch_bytes) {
+  ContrastiveGeom g{};
+  if (int r = contrastive_geometry(cfg, &g)) return r;
+  if (!saved_bytes || !scratch_bytes) return fail(GLOM_B200_ERR_INVALID, "contrastive: output pointer is NULL");
+  const ContrastiveLayout w = contrastive_layout(g);
+  *saved_bytes = w.saved;
+  *scratch_bytes = w.scratch;
+  return 0;
+}
+
+GLOM_B200_API int glom_b200_contrastive_forward(const glom_b200_contrastive_cfg* cfg, const float* za, const float* zb,
+                                                float* loss, void* saved, size_t saved_bytes, void* scratch,
+                                                size_t scratch_bytes, void* stream) {
+  ContrastiveGeom g{};
+  if (int r = contrastive_geometry(cfg, &g)) return r;
+  if (!za || !zb || !loss || !saved || !scratch) return fail(GLOM_B200_ERR_INVALID, "contrastive forward: a pointer is NULL");
+  const ContrastiveLayout w = contrastive_layout(g);
+  if (saved_bytes < w.saved || scratch_bytes < w.scratch)
+    return fail(GLOM_B200_ERR_WORKSPACE, "contrastive forward: need %zu saved / %zu scratch bytes, got %zu / %zu", w.saved,
+                w.scratch, saved_bytes, scratch_bytes);
+  if (reinterpret_cast<uintptr_t>(saved) % 1024 || reinterpret_cast<uintptr_t>(scratch) % 1024)
+    return fail(GLOM_B200_ERR_INVALID, "contrastive forward: saved and scratch must be 1024-byte aligned");
+  DeviceInfo di{};
+  if (int r = device_info(&di)) return r;
+  if (int r = bind_current_device()) return r;
+  g_launches = 0;
+  if (contrastive_forward(g, za, zb, loss, saved, scratch, g_encode, di.sms, static_cast<cudaStream_t>(stream), &g_launches,
+                          g_err, sizeof(g_err)))
+    return GLOM_B200_ERR_CUDA;
+  return 0;
+}
+
+GLOM_B200_API int glom_b200_contrastive_backward(const glom_b200_contrastive_cfg* cfg, const float* za, const float* zb,
+                                                 const float* grad_loss, const void* saved, size_t saved_bytes, float* dza,
+                                                 float* dzb, void* stream) {
+  ContrastiveGeom g{};
+  if (int r = contrastive_geometry(cfg, &g)) return r;
+  if (!za || !zb || !grad_loss || !saved || !dza || !dzb)
+    return fail(GLOM_B200_ERR_INVALID, "contrastive backward: a pointer is NULL");
+  if (dza == dzb || (const float*)dza == za || (const float*)dza == zb || (const float*)dzb == za || (const float*)dzb == zb)
+    return fail(GLOM_B200_ERR_INVALID, "contrastive backward: dza / dzb must not alias the inputs or each other");
+  const ContrastiveLayout w = contrastive_layout(g);
+  if (saved_bytes < w.saved) return fail(GLOM_B200_ERR_WORKSPACE, "contrastive backward: need %zu saved bytes, got %zu", w.saved, saved_bytes);
+  if (reinterpret_cast<uintptr_t>(saved) % 1024 || reinterpret_cast<uintptr_t>(dza) % 16 || reinterpret_cast<uintptr_t>(dzb) % 16)
+    return fail(GLOM_B200_ERR_INVALID, "contrastive backward: saved must be 1024-byte, dza / dzb 16-byte aligned");
+  DeviceInfo di{};
+  if (int r = device_info(&di)) return r;
+  if (int r = bind_current_device()) return r;
+  g_launches = 0;
+  if (contrastive_backward(g, za, zb, grad_loss, saved, dza, dzb, g_encode, static_cast<cudaStream_t>(stream), &g_launches,
+                           g_err, sizeof(g_err)))
+    return GLOM_B200_ERR_CUDA;
+  return 0;
+}
+
 GLOM_B200_API int glom_b200_clock_probe(uint64_t* out_cycles_ns, int spin_us, void* stream) {
   if (!out_cycles_ns || spin_us < 1 || spin_us > 100000) return fail(GLOM_B200_ERR_INVALID, "clock probe: bad arguments");
   cudaError_t e = launch_clock_probe(reinterpret_cast<unsigned long long*>(out_cycles_ns), (unsigned long long)spin_us * 1000ull,

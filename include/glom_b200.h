@@ -202,6 +202,44 @@ GLOM_B200_API int glom_b200_islands(const float* states, int slabs, int side_h, 
                                     float* cos_right, float* cos_down, float* agreement, int32_t* labels,
                                     int32_t* num_islands, void* stream);
 
+/* Column-contrastive loss on selected levels of two views (the regulariser the reference's README lists as its open Todo,
+ * "contrastive / consistency regularization of top-ish levels"; DESIGN section 9).  za, zb: (B, n, L, d) fp32 with d
+ * contiguous and element strides given in the cfg.  Per selected level, rows r = (b, i), R = B n of them:
+ *   a_r = za[b,i,l] / max(|za[b,i,l]|, 1e-12), b_r likewise;  s_rc = <a_r, b_c> / tau;
+ *   candidates of r: {r} and every column of another image;
+ *   l_r = 1/2 [ (lse_(c in cand r) s_rc - s_rr) + (lse_(c in cand r) s_cr - s_rr) ];  loss = mean over levels and rows.
+ * tcgen05 kernels: bf16 unit vectors as GEMM operands, fp32 accumulation, fp32 softmax sums and gradients; no buffer of
+ * R x R (or R x R / 128) elements exists.  Requires dim % 64 == 0, temperature >= 0.03 (then 1/tau is a valid fixed
+ * stabiliser: 2 log2(e) / tau <= 96), 1 <= num_selected <= 32 distinct levels.  No atomics: results are bit-reproducible. */
+#define GLOM_B200_CONTRASTIVE_MAX_LEVELS 32
+typedef struct glom_b200_contrastive_cfg {
+  uint32_t struct_size;   /* = sizeof(glom_b200_contrastive_cfg)                                  */
+  int32_t batch, n, levels, dim;
+  int32_t num_selected;   /* entries of `selected` in use                                          */
+  int32_t selected[GLOM_B200_CONTRASTIVE_MAX_LEVELS];   /* level indices in [0, levels), distinct  */
+  float temperature;      /* tau >= 0.03                                                           */
+  int64_t stride_a[3];    /* element strides of za over (B, n, L); d has stride 1                  */
+  int64_t stride_b[3];
+} glom_b200_contrastive_cfg;
+
+/* Bytes of the two caller-owned buffers (no device needed; both grow linearly in B n):
+ *   saved:   what the backward reads (bf16 unit rows of both views, per-row fp32 norms / lse / diagonal terms); it must
+ *            stay untouched from _forward until _backward of the same loss.  1024-byte aligned.
+ *   scratch: forward-only (lse partial sums, loss partials); may be reused as soon as _forward's work has run.
+ * GLOM_B200_ERR_INVALID for an unsupported cfg (dim % 64 != 0, tau < 0.03, bad level list, ...). */
+GLOM_B200_API int glom_b200_contrastive_workspace_bytes(const glom_b200_contrastive_cfg* cfg, size_t* saved_bytes,
+                                                        size_t* scratch_bytes);
+/* loss: one fp32 device word, overwritten (not accumulated).  za / zb may alias each other. */
+GLOM_B200_API int glom_b200_contrastive_forward(const glom_b200_contrastive_cfg* cfg, const float* za, const float* zb,
+                                                float* loss, void* saved, size_t saved_bytes, void* scratch,
+                                                size_t scratch_bytes, void* stream);
+/* grad_loss: one fp32 device word (dL/dloss; read on the device, no host synchronisation).  dza, dzb: (B, n, L, d)
+ * contiguous fp32, OVERWRITTEN with the full gradients (exact zeros at unselected levels); must not alias za, zb or each
+ * other.  `saved` as filled by the matching _forward. */
+GLOM_B200_API int glom_b200_contrastive_backward(const glom_b200_contrastive_cfg* cfg, const float* za, const float* zb,
+                                                 const float* grad_loss, const void* saved, size_t saved_bytes, float* dza,
+                                                 float* dzb, void* stream);
+
 /* Measurement aid (bench.py): one device thread spins for `spin_us` microseconds of %globaltimer and writes
  * {SM cycles elapsed, nanoseconds elapsed} to out_cycles_ns[0..1] (device memory, 16 bytes): cycles / ns is the SM
  * clock in GHz the device actually ran at when the probe executed.  Enqueued on `stream`; the caller synchronises. */
